@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — IMPALA env-steps/s on synthetic Atari-shaped envs (BASELINE.json metric).
 
-    python bench.py [--gpus N --steps K --warmup W] [--impl reference]
+    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" = one full actor-learner iteration of the hot path: T=50 lock-step env steps of the whole
@@ -45,7 +45,12 @@ def parse():
     ap.add_argument('--ref-deepmind-seconds', type=float, default=20.0,
                     help='--impl reference: extra run of the full wrap_deepmind pipeline flavour (0 = skip)')
     ap.add_argument('--no-pipeline', action='store_true', help='strictly sequential rollout -> learn')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed (rank 0) to DIR/<name>.npy, float32, at most 64 MB')
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs dumps the timed path of --impl ours')
+    return args
 
 
 class ClockSampler(object):
@@ -226,6 +231,9 @@ def main():
         losses = step()
     ev1.record()
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        # before the untimed K1 steps below overwrite the engine's buffers and weights
+        dump_outputs(eng, losses, args.dump_outputs)
     if world > 1:
         dist.barrier()
     elapsed_ms = torch.tensor([ev0.elapsed_time(ev1)], device=dev)
@@ -403,6 +411,40 @@ def main():
         dist.destroy_process_group()
 
 
+DUMP_ENV_COLUMNS = 2048                   # env columns kept of each (T, B, ...) buffer: 36 MB in all at 4096 envs
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(eng, losses, out_dir):
+    """What the last timed step computed, as float32 .npy files: the losses step() returned, the weights after its
+    update, the rollout the update trained on with the learner's logits and values for it, and (pipelined engines)
+    the rollout produced alongside it.  The (T, B, ...) buffers keep a fixed, seeded sample of env columns, so
+    that two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    import torch
+    B = eng.B
+    cols = torch.from_numpy(np.sort(np.random.default_rng(0).choice(B, min(B, DUMP_ENV_COLUMNS), replace=False)))
+
+    def sample(t):
+        return t[:, cols.to(t.device)].float().cpu().numpy()
+
+    def rollout(st, prefix):
+        return {prefix + 'actions': sample(st['actions']), prefix + 'behaviour_logits': sample(st['beh_logits']),
+                prefix + 'rewards': sample(st['rewards']), prefix + 'dones': sample(st['dones'])}
+
+    out = dict(losses=losses.float().cpu().numpy(),
+               params=torch.cat([p.detach().reshape(-1) for p in eng.model.parameters()]).float().cpu().numpy(),
+               learner_logits=sample(eng.tgt_logits), learner_values=sample(eng.values))
+    out.update(rollout(eng._sets[eng._cur_set], ''))
+    if eng.pipeline:
+        out.update(rollout(eng._sets[1 - eng._cur_set], 'next_'))
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_MAX_BYTES, 'dump of %d bytes exceeds %d' % (total, DUMP_MAX_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 # dram__bytes_read.sum + dram__bytes_write.sum per sample of conv1 forward from the committed ncu captures:
 # bf16 input (profiles/r01_learner_kernels_final.txt: 2.948 GB + 1.282 GB at 51 200 samples); uint8 input
 # (profiles/r02_conv1_u8_ncu.txt: 1.445 GB + 1.270 GB)
@@ -530,7 +572,7 @@ def run_e2e(eng, args, world, dev):
     if world > 1:
         agent.alg.grad_sync = lambda g: dist.all_reduce(g, op=dist.ReduceOp.SUM)
     actor = Actor(cfg, device=dev)
-    steps = max(10, min(args.steps, 20))
+    steps = args.steps
     actor.set_weights(agent.get_weights()).get()
     fut = actor.sample()
 
