@@ -499,6 +499,48 @@ int rl_rollout_mlp(int n_layers, const int* dims, int n_seg, const int* seg_laye
                    float* val_out, float* logits_out, float* rew_out, uint8_t* done_out,
                    double* const* vecnorm_state, const double* vecnorm_cfg, int vecnorm_flags, rl_stream_t stream);
 
+/* ------------------------------------------------------------------------
+ * Off-policy continuous control (DDPG / TD3 / SAC).  Replaces the per-step loop of
+ * benchmark/torch/{td3,sac,ddpg}/train.py: agent.sample -> env.step -> rpm.append -> rpm.sample_batch.
+ *
+ * rl_explore_mlp: ONE launch runs K lock-step steps of B MuJoCo-shaped synthetic envs (the env of
+ *   rl_env_mujoco_synth_step): actor forward, exploration rule, env step, episode bookkeeping, and writes every
+ *   transition straight into the rows of a replay ring of rm_max_size rows:
+ *     rm_obs / rm_next_obs [cap, obs_dim] f32, rm_action [cap, action_dim] f32, rm_reward [cap] f32,
+ *     rm_terminal [cap] i32.  Step t of env b goes to row (rm_pos + t*B + b) % rm_max_size (the order of K
+ *     successive batch appends); K*B > rm_max_size is rejected (a launch would overwrite its own rows).
+ *   Actor: n_layers-1 (1..3) ReLU hidden layers and a head, fp32 parameters read in place (row segments as in
+ *     rl_mlp_fwd; widths <= 512); head 0: tanh(out) [action_dim] (TD3 / DDPG), head 1: out = [mean | log_std]
+ *     [2*action_dim], log_std clamped to [-20, 2] (SAC).  The actor is not evaluated in mode 0.
+ *   mode 0 (warm-up): a = 2u - 1, u = 24-bit uniform word (d % 4) of philox(env, step, d / 4, STREAM_ACTION);
+ *   mode 1 (deterministic + noise, head 0): a = clip(tanh(out) + expl_noise * z, -1, 1), z Gaussian on STREAM_GAUSS
+ *     (expl_noise = 0 is the deterministic policy);
+ *   mode 2 (SAC, head 1): a = tanh(mean + exp(log_std) * z).
+ *   Env: reward / done from STREAM_REWDONE at (env, step), next observation at step + 1 on STREAM_OBS; done also at
+ *     the time limit (max_episode_steps > 0); terminal = done and not the time-limit step.  The env auto-resets: the
+ *     next_obs of a done step is the first observation of the next episode (terminal rows mask it by 1 - terminal).
+ *   obs_cur [B, obs_dim] in/out carries the observations between launches; step index of row t = step0 + t.
+ *   The rows of every layer are split over a thread-block cluster of up to 8 CTAs that keeps the actor resident in
+ *   shared memory for all K steps; an actor that does not fit 8 CTAs is rejected.
+ *
+ * rl_replay_sample_uniform: n rows drawn uniformly from the first min(*size_dev, capacity) rows of a ring of
+ *   `capacity` rows, gathered densely:
+ *   obs_out / next_obs_out [n, obs_dim], action_out [n, act_dim], reward_out / terminal_out [n] (f32), idx_out [n]
+ *   (optional).  Row i of draw d = *draw_dev is (x * size) >> 32, x = word 0 of philox(i, d, 0, STREAM_REPLAY).
+ *   size and draw are read from device memory, so a captured graph draws fresh rows on every replay. */
+int rl_explore_mlp(int n_layers, const int* dims, int n_seg, const int* seg_layer, const int* seg_rows,
+                   const float* const* seg_w, const float* const* seg_b, int head, int mode, int K, int B,
+                   int action_dim, float expl_noise, float* obs_cur, float* ep_ret, int32_t* ep_len, float* totals,
+                   float* ring_ret, int32_t* ring_len, uint32_t* ring_head, int ring_cap, uint64_t seed,
+                   uint32_t step0, uint32_t env_offset, float p_done, int max_episode_steps, float* rm_obs,
+                   float* rm_action, float* rm_reward, int32_t* rm_terminal, float* rm_next_obs, int rm_max_size,
+                   int rm_pos, rl_stream_t stream);
+int rl_replay_sample_uniform(const float* obs, const float* action, const float* reward, const int32_t* terminal,
+                             const float* next_obs, int obs_dim, int act_dim, const int32_t* size_dev,
+                             const int32_t* draw_dev, int capacity, int n, uint64_t seed, float* obs_out, float* action_out,
+                             float* reward_out, float* terminal_out, float* next_obs_out, int32_t* idx_out,
+                             rl_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -95,6 +95,11 @@ SIGNATURES = {
     'rl_rollout_mlp': (c_i, [c_i, c_p, c_i, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_i, c_p, c_p,
                              c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_u64, c_u32, c_u32, c_f, c_i, c_p, c_p, c_p, c_p, c_p,
                              c_p, c_p, c_p, c_p, c_i, c_p]),
+    'rl_explore_mlp': (c_i, [c_i, c_p, c_i, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_f, c_p, c_p, c_p, c_p,
+                             c_p, c_p, c_p, c_i, c_u64, c_u32, c_u32, c_f, c_i, c_p, c_p, c_p, c_p, c_p, c_i, c_i,
+                             c_p]),
+    'rl_replay_sample_uniform': (c_i, [c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_p, c_p, c_i, c_i, c_u64, c_p, c_p, c_p, c_p,
+                                       c_p, c_p, c_p]),
     'rl_mask_scatter_grid_bf16': (c_i, [c_p, c_p, c_p, ctypes.c_longlong, c_i, c_i, c_i, c_i, c_i, c_p]),
 }
 

@@ -215,3 +215,131 @@ class AtariQModel(Model):
             v = self.linear_2_val(F.relu(self.linear_1_val(x)))
             return a + (v - a.mean(dim=1, keepdim=True))
         return self.linear_1(x)
+
+
+# ---- continuous-control actor / critic pairs (benchmark/torch/{td3,sac,ddpg}/mujoco_model.py), torch default init ----
+class _TwinCritic(Model):
+    """Two 256-256 ReLU Q networks on cat(obs, action) (td3 / sac mujoco_model.py Critic)."""
+
+    def __init__(self, obs_dim, act_dim):
+        super(_TwinCritic, self).__init__()
+        self.l1, self.l2, self.l3 = nn.Linear(obs_dim + act_dim, 256), nn.Linear(256, 256), nn.Linear(256, 1)
+        self.l4, self.l5, self.l6 = nn.Linear(obs_dim + act_dim, 256), nn.Linear(256, 256), nn.Linear(256, 1)
+
+    def forward(self, obs, action):
+        sa = torch.cat([obs, action], 1)
+        q1 = self.l3(F.relu(self.l2(F.relu(self.l1(sa)))))
+        q2 = self.l6(F.relu(self.l5(F.relu(self.l4(sa)))))
+        return q1, q2
+
+    def Q1(self, obs, action):
+        sa = torch.cat([obs, action], 1)
+        return self.l3(F.relu(self.l2(F.relu(self.l1(sa)))))
+
+
+class _TanhActor(Model):
+    """ReLU MLP with a tanh head (td3 / ddpg mujoco_model.py Actor)."""
+
+    def __init__(self, obs_dim, act_dim, h1, h2):
+        super(_TanhActor, self).__init__()
+        self.l1, self.l2, self.l3 = nn.Linear(obs_dim, h1), nn.Linear(h1, h2), nn.Linear(h2, act_dim)
+
+    def forward(self, obs):
+        return torch.tanh(self.l3(F.relu(self.l2(F.relu(self.l1(obs))))))
+
+
+class _GaussianActor(Model):
+    """sac/mujoco_model.py Actor: 256-256 ReLU trunk, mean and log-std heads, log-std clamped to [-20, 2]."""
+
+    def __init__(self, obs_dim, act_dim):
+        super(_GaussianActor, self).__init__()
+        self.l1, self.l2 = nn.Linear(obs_dim, 256), nn.Linear(256, 256)
+        self.mean_linear, self.std_linear = nn.Linear(256, act_dim), nn.Linear(256, act_dim)
+
+    def forward(self, obs):
+        x = F.relu(self.l2(F.relu(self.l1(obs))))
+        return self.mean_linear(x), torch.clamp(self.std_linear(x), min=-20.0, max=2.0)
+
+
+class _DDPGCritic(Model):
+    """ddpg/mujoco_model.py Critic: obs -> 400 (ReLU), cat action -> 300 (ReLU) -> 1."""
+
+    def __init__(self, obs_dim, act_dim):
+        super(_DDPGCritic, self).__init__()
+        self.l1, self.l2, self.l3 = nn.Linear(obs_dim, 400), nn.Linear(400 + act_dim, 300), nn.Linear(300, 1)
+
+    def forward(self, obs, action):
+        q = F.relu(self.l1(obs))
+        return self.l3(F.relu(self.l2(torch.cat([q, action], 1))))
+
+
+class _ActorCriticModel(Model):
+    def policy(self, obs):
+        return self.actor_model(obs)
+
+    def value(self, obs, action):
+        return self.critic_model(obs, action)
+
+    def get_actor_params(self):
+        return self.actor_model.parameters()
+
+    def get_critic_params(self):
+        return self.critic_model.parameters()
+
+
+class TD3MujocoModel(_ActorCriticModel):
+    """benchmark/torch/td3/mujoco_model.py: actor 17 -> 256 -> 256 -> act (tanh), twin 256-256 critics."""
+
+    def __init__(self, obs_space=17, act_space=6):
+        super(TD3MujocoModel, self).__init__()
+        obs_dim, act_dim = _dim(obs_space), _dim(act_space)
+        self.actor_model = _TanhActor(obs_dim, act_dim, 256, 256)
+        self.critic_model = _TwinCritic(obs_dim, act_dim)
+
+    def Q1(self, obs, action):
+        return self.critic_model.Q1(obs, action)
+
+    def native_actor_layers(self):
+        """Row segments per linear layer of the actor for rl_explore_mlp (ReLU hidden layers, tanh head)."""
+        from ..kernels import ACT_RELU, HEAD_TANH
+        a = self.actor_model
+        return [[(a.l1.weight, a.l1.bias)], [(a.l2.weight, a.l2.bias)], [(a.l3.weight, a.l3.bias)]], ACT_RELU, HEAD_TANH
+
+
+class SACMujocoModel(_ActorCriticModel):
+    """benchmark/torch/sac/mujoco_model.py: actor 17 -> 256 -> 256 -> {mean, log-std}, twin 256-256 critics."""
+
+    def __init__(self, obs_space=17, act_space=6):
+        super(SACMujocoModel, self).__init__()
+        obs_dim, act_dim = _dim(obs_space), _dim(act_space)
+        self.actor_model = _GaussianActor(obs_dim, act_dim)
+        self.critic_model = _TwinCritic(obs_dim, act_dim)
+
+    def Q1(self, obs, action):
+        return self.critic_model.Q1(obs, action)
+
+    def native_actor_layers(self):
+        """Head outputs = [mean (act_dim) | log-std (act_dim)] (the kernel applies the clamp)."""
+        from ..kernels import ACT_RELU, HEAD_MEAN_LOGSTD
+        a = self.actor_model
+        return [[(a.l1.weight, a.l1.bias)], [(a.l2.weight, a.l2.bias)],
+                [(a.mean_linear.weight, a.mean_linear.bias), (a.std_linear.weight, a.std_linear.bias)]], \
+            ACT_RELU, HEAD_MEAN_LOGSTD
+
+
+class DDPGMujocoModel(_ActorCriticModel):
+    """benchmark/torch/ddpg/mujoco_model.py: actor 17 -> 400 -> 300 -> act (tanh), critic 400 / 300."""
+
+    def __init__(self, obs_space=17, act_space=6):
+        super(DDPGMujocoModel, self).__init__()
+        obs_dim, act_dim = _dim(obs_space), _dim(act_space)
+        self.actor_model = _TanhActor(obs_dim, act_dim, 400, 300)
+        self.critic_model = _DDPGCritic(obs_dim, act_dim)
+
+    def Q1(self, obs, action):
+        return self.critic_model(obs, action)
+
+    def native_actor_layers(self):
+        from ..kernels import ACT_RELU, HEAD_TANH
+        a = self.actor_model
+        return [[(a.l1.weight, a.l1.bias)], [(a.l2.weight, a.l2.bias)], [(a.l3.weight, a.l3.bias)]], ACT_RELU, HEAD_TANH

@@ -704,6 +704,8 @@ def mask_scatter_grid_bf16(src, act, dst, n, PH, PW, GH, GW, C):
 
 # --------------------------------------------------------------------------- fused fp32 MLP (K6, MLP model family)
 ACT_RELU, ACT_TANH, ACT_NONE = 0, 1, 2
+HEAD_TANH, HEAD_MEAN_LOGSTD = 0, 1                       # rl_explore_mlp actor heads
+EXPLORE_WARMUP, EXPLORE_NOISE, EXPLORE_SAC = 0, 1, 2     # rl_explore_mlp exploration rules
 
 
 class MlpPlan(object):
@@ -816,6 +818,83 @@ class MlpPlan(object):
                                          vecnorm.c_state if vecnorm is not None else None,
                                          vecnorm.c_cfg if vecnorm is not None else None,
                                          vecnorm.flags if vecnorm is not None else 0, stream()), 'rollout_mlp')
+
+    def explore(self, memory, mode, K, obs_cur, stats, seed, step0, head=HEAD_TANH, expl_noise=0.1, env_offset=0,
+                p_done=0.01, max_episode_steps=1000):
+        """rl_explore_mlp: K lock-step steps of B = obs_cur.shape[0] envs in ONE launch (actor forward + exploration
+        rule + env step), transitions written into ``memory`` (a utils.ReplayMemory) at rows
+        (memory._curr_pos + t*B + b) % memory.max_size.  The caller advances the memory with ``memory.commit(K*B)``."""
+        if self.act != ACT_RELU:
+            raise RuntimeError('parl_b200: explore needs ReLU hidden layers (act %d)' % self.act)
+        if head not in (HEAD_TANH, HEAD_MEAN_LOGSTD):
+            raise RuntimeError('parl_b200: explore head must be HEAD_TANH or HEAD_MEAN_LOGSTD, got %r' % (head, ))
+        if int(mode) not in (EXPLORE_WARMUP, EXPLORE_NOISE, EXPLORE_SAC):
+            raise RuntimeError('parl_b200: explore mode must be 0, 1 or 2, got %r' % (mode, ))
+        if int(mode) == EXPLORE_NOISE and head != HEAD_TANH:
+            raise RuntimeError('parl_b200: explore mode 1 needs the tanh head')
+        if int(mode) == EXPLORE_SAC and head != HEAD_MEAN_LOGSTD:
+            raise RuntimeError('parl_b200: explore mode 2 needs the mean|log-std head')
+        AD = self.out_dim if head == HEAD_TANH else self.out_dim // 2
+        D = self.dims_list[0]
+        m = memory
+        require_cuda(obs_cur, m.obs, m.action, m.reward, m.terminal, m.next_obs)
+        if obs_cur.dim() != 2 or obs_cur.shape[1] != D:
+            raise RuntimeError('parl_b200: obs_cur must be [B, %d], got %s' % (D, tuple(obs_cur.shape)))
+        B, cap = obs_cur.shape[0], m.max_size
+        _chk('obs_cur', obs_cur, torch.float32, B * D)
+        _chk('memory.obs', m.obs, torch.float32, cap * D)
+        _chk('memory.next_obs', m.next_obs, torch.float32, cap * D)
+        _chk('memory.action', m.action, torch.float32, cap * AD)
+        _chk('memory.reward', m.reward, torch.float32, cap)
+        _chk('memory.terminal', m.terminal, torch.int32, cap)
+        _chk('stats.ep_len', stats.ep_len, torch.int32, B)
+        if int(K) < 1 or int(K) * B > cap:
+            raise RuntimeError('parl_b200: explore K*B = %d transitions must be in 1..%d (the replay capacity)'
+                               % (int(K) * B, cap))
+        check(_lib.load().rl_explore_mlp(self.n_layers, self.c_dims, len(self.segs), self.c_layer, self.c_rows, self.c_w,
+                                         self.c_b, int(head), int(mode), int(K), B, AD, float(expl_noise), ptr(obs_cur),
+                                         *stats.args(), int(seed), int(step0), int(env_offset), float(p_done),
+                                         int(max_episode_steps), ptr(m.obs), ptr(m.action), ptr(m.reward),
+                                         ptr(m.terminal), ptr(m.next_obs), cap, int(m._curr_pos), stream()),
+              'explore_mlp')
+
+
+def replay_sample_uniform(memory, n, size_dev, draw_dev, seed, out=None, want_idx=False):
+    """rl_replay_sample_uniform: n uniform rows of the first min(size_dev[0], memory.max_size) rows of ``memory`` (a
+    utils.ReplayMemory with float actions) -> (obs, action, reward [n], next_obs, terminal [n]) float32 device tensors
+    (``out``: the same tuple preallocated), plus the int32 rows with ``want_idx``.  size_dev / draw_dev: int32 [1]
+    device tensors."""
+    m = memory
+    require_cuda(m.obs, m.action, m.reward, m.terminal, m.next_obs, size_dev, draw_dev)
+    cap, D = m.obs.shape
+    AD = m.action.shape[1]
+    _chk('memory.obs', m.obs, torch.float32, cap * D)
+    _chk('memory.next_obs', m.next_obs, torch.float32, cap * D)
+    _chk('memory.action', m.action, torch.float32, cap * AD)
+    _chk('memory.reward', m.reward, torch.float32, cap)
+    _chk('memory.terminal', m.terminal, torch.int32, cap)
+    _chk('size_dev', size_dev, torch.int32, 1)
+    _chk('draw_dev', draw_dev, torch.int32, 1)
+    n = int(n)
+    if n < 1:
+        raise RuntimeError('parl_b200: replay_sample_uniform needs n >= 1, got %d' % n)
+    dev = m.obs.device
+    if out is None:
+        f32 = torch.float32
+        out = (torch.empty((n, D), dtype=f32, device=dev), torch.empty((n, AD), dtype=f32, device=dev),
+               torch.empty(n, dtype=f32, device=dev), torch.empty((n, D), dtype=f32, device=dev),
+               torch.empty(n, dtype=f32, device=dev))
+    obs, act, rew, nobs, term = out
+    require_cuda(obs, act, rew, nobs, term)
+    for nm, t, k in (('obs', obs, n * D), ('action', act, n * AD), ('reward', rew, n), ('next_obs', nobs, n * D),
+                     ('terminal', term, n)):
+        _chk(nm, t, torch.float32, k)
+    idx = torch.empty(n, dtype=torch.int32, device=dev) if want_idx else None
+    check(_lib.load().rl_replay_sample_uniform(ptr(m.obs), ptr(m.action), ptr(m.reward), ptr(m.terminal),
+                                               ptr(m.next_obs), D, AD, ptr(size_dev), ptr(draw_dev), cap, n, int(seed),
+                                               ptr(obs), ptr(act), ptr(rew), ptr(term), ptr(nobs), ptr(idx), stream()),
+          'replay_sample_uniform')
+    return (obs, act, rew, nobs, term, idx) if want_idx else (obs, act, rew, nobs, term)
 
 
 ENV_MUJOCO_SYNTH, ENV_CARTPOLE = 0, 1

@@ -54,6 +54,15 @@ class ReplayMemory(object):
         self._curr_size = min(self._curr_size + n, self.max_size)
         self._curr_pos = (self._curr_pos + n) % self.max_size
 
+    def commit(self, n):
+        """Account for n rows a device kernel wrote in place from the current position on (rl_explore_mlp): the same
+        bookkeeping as ``append_batch`` of n transitions."""
+        n = int(n)
+        if n < 0 or n > self.max_size:
+            raise ValueError('ReplayMemory.commit: n=%d outside 0..%d' % (n, self.max_size))
+        self._curr_size = min(self._curr_size + n, self.max_size)
+        self._curr_pos = (self._curr_pos + n) % self.max_size
+
     # ---- reads ------------------------------------------------------------------------------------------
     def make_index(self, batch_size):
         return np.random.randint(self._curr_size, size=batch_size)
